@@ -3,6 +3,7 @@
 metric), through the drop-in modules -> libffc_b200.so.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--math fp32|bf16x3]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one forward pass of the generator over one batch of 32 synthetic 512x512 (image, mask)
@@ -18,6 +19,9 @@ Reported on one JSON line by rank 0:
                with SURVEY.md §8(d)'s algorithmic bytes
   cpu_baseline the oracle's torch-CPU port (the reference's own operator sequence) on this box's host cores
 `--impl reference` times that CPU port alone (bounded sample per step) as the reference arm.
+
+--dump-outputs DIR writes what the timed paths returned in their last step (rank 0's shard), so that two builds can
+be compared output for output: weights and inputs are seeded, identical from run to run for the same arguments.
 """
 import argparse
 import json
@@ -116,7 +120,7 @@ def cpu_reference_step(images, threads=None):
     x = st["x"][:images]
     t0 = time.perf_counter()
     with torch.no_grad():
-        otc.ffc_resnet_generator(x, st["sd"], **BIG_LAMA_KWARGS)
+        st["y"] = otc.ffc_resnet_generator(x, st["sd"], **BIG_LAMA_KWARGS)
     return time.perf_counter() - t0, images
 
 
@@ -249,6 +253,26 @@ def torch_cuda_baseline(dev, B, S, steps=5, warmup=3):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array (name -> CPU tensor) as DIR/<name>.npy in float32.  The arrays share DUMP_BYTES: one larger
+    than its share is replaced by a fixed seeded sample of its elements (the same positions in every run of the same
+    shape), whose flat indices go to DIR/<name>_index.npy as float64 (exact below 2**53)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096                  # room for the .npy headers
+    for name, t in arrays.items():
+        a = np.ascontiguousarray(t.numpy(), dtype=np.float32)
+        if a.nbytes > share:
+            k = share // 12                                   # 4 bytes of value + 8 of index per sampled element
+            idx = np.sort(np.random.default_rng(0).choice(a.size, k, replace=False, shuffle=False))
+            np.save(os.path.join(dirname, name + "_index.npy"), idx.astype(np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def run_reference(args, rank, world, out):
     """Reference arm: the reference's CPU path (oracle torch-CPU port; the reference tree itself cannot
     travel to the GPU box) on all host threads.  Rank 0 only."""
@@ -262,6 +286,8 @@ def run_reference(args, rank, world, out):
     for _ in range(args.steps):
         dt, _n = cpu_reference_step(per_step)
         t += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"y": cpu_reference_step.state["y"]})
     v = per_step * args.steps / t
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": "images/s", "n_gpus": args.gpus,
@@ -304,7 +330,12 @@ def main():
                     help="skip the torch-eager (cuFFT/cuDNN) reading of the same operator sequence on this GPU")
     ap.add_argument("--io", default=os.environ.get("LAMA_B200_BENCH_IO", "both"), choices=["f32", "both"],
                     help="both: also time the uint8 predict path (lama_b200.predict, SURVEY.md row f1) end to end")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of each timed path's last step to DIR/<name>.npy "
+                         "(float32, at most 64 MB in all: larger outputs are sampled at fixed seeded positions)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -382,6 +413,10 @@ def main():
         ms = timed(graphed.graph.replay, args.steps)
     clocks = clk.summary()
     value = world * B * args.steps / (ms / 1e3)
+    # what each timed path returned in its last step, copied before later work reuses its buffers
+    dumps, dump = {}, bool(args.dump_outputs) and rank == 0
+    if dump:
+        dumps["y"] = ex.outputs["y0"].cpu()
 
     # ---- end to end through the public serving API with HOST buffers: every step copies its pinned (B,4,S,S)
     # input to the device and its (B,3,S,S) result back; GeneratorPipeline overlaps those copies with the
@@ -403,6 +438,8 @@ def main():
     pipe.drain()
     barrier()
     ms_e2e = (_time.perf_counter() - t0) * 1e3
+    if dump:
+        dumps["e2e_y"] = y_host.clone()
     if world > 1:
         t = torch.tensor([ms_e2e], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -571,6 +608,8 @@ def main():
             pipe8.drain()
             barrier()
             ms8 = (_time.perf_counter() - t0) * 1e3
+            if dump:
+                dumps["u8_io_y"] = y8.float()
             if world > 1:
                 t = torch.tensor([ms8], device=dev)
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -582,6 +621,8 @@ def main():
         except Exception as ex_u8:  # noqa: BLE001
             u8_io = {"error": f"{type(ex_u8).__name__}: {ex_u8}"[:300]}
 
+    if dump:
+        dump_outputs(args.dump_outputs, dumps)
     if rank == 0:
         print(json.dumps({
             "metric": METRIC, "value": value, "unit": "images/s", "n_gpus": world, "steps": args.steps,

@@ -222,12 +222,47 @@ def make_f4():
     _save("resblock_64_lfu_8x8", x_l=xl.numpy(), x_g=xg.numpy(), y_l=yl.numpy(), y_g=yg.numpy(), **_sd_np(m))
 
 
+def _sd_fingerprint(module):
+    """state_dict schema (every key, num_batches_tracked included, with its shape) and one float64 sum per tensor:
+    enough to show that ``seeded_parameters_`` gives a drop-in module the reference's values under the same keys,
+    without storing the weights."""
+    import json
+    sd = module.state_dict()
+    return dict(sd_schema=np.asarray(json.dumps({k: list(v.shape) for k, v in sd.items()})),
+                sd_sums=np.asarray([v.double().sum().item() for v in sd.values()]))
+
+
+@torch.no_grad()
+def make_surface():
+    """Module surface kept identical to the reference beyond the generator: the FFC_BN_ACT torch composition with
+    LFU (the CPU / unsupported-option path) and FFCNLayerDiscriminator (ffc.py:370-433, training only)."""
+    ffc = load_reference_ffc()
+    torch.set_num_threads(1)
+    kw = dict(in_channels=32, out_channels=32, kernel_size=3, ratio_gin=0.75, ratio_gout=0.75, padding=1,
+              activation_layer=torch.nn.ReLU, enable_lfu=True)
+    m = seeded_parameters_(ffc.FFC_BN_ACT(**kw).eval(), 5)
+    xl, xg = _randn((1, 8, 8, 8), 800), _randn((1, 24, 8, 8), 801)
+    yl, yg = m((xl, xg))
+    _save("surface_ffcbnact_32_k3_lfu_8x8", x_l=xl.numpy(), x_g=xg.numpy(), y_l=yl.numpy(), y_g=yg.numpy(),
+          **_sd_fingerprint(m))
+    kw = dict(input_nc=3, ndf=16, n_layers=3, init_conv_kwargs=dict(ratio_gin=0, ratio_gout=0.5, enable_lfu=False),
+              conv_kwargs=dict(ratio_gin=0.5, ratio_gout=0.5, enable_lfu=False))
+    m = seeded_parameters_(ffc.FFCNLayerDiscriminator(**kw).eval(), 9)
+    x = _randn((1, 3, 32, 32), 1)
+    y, feats = m(x)
+    _save("surface_discriminator_ndf16_32x32", x=x.numpy(), y=y.numpy(),
+          **{f"feat{i}": f.numpy() for i, f in enumerate(feats)}, **_sd_fingerprint(m))
+
+
 if __name__ == "__main__":
     if "--f4-only" in sys.argv:
         make_f4()
     elif "--predict-only" in sys.argv:
         make_predict()
+    elif "--surface-only" in sys.argv:
+        make_surface()
     else:
         main()
         make_predict()
         make_f4()
+        make_surface()

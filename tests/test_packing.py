@@ -4,10 +4,10 @@ import json
 import os
 
 import numpy as np
-import pytest
 import torch
 import torch.nn.functional as F
 
+from conftest import load_golden
 from lama_b200 import _lib as L
 from lama_b200 import modules as M
 from lama_b200 import packing as P
@@ -75,39 +75,42 @@ def test_state_dict_schema_matches_reference():
     assert isinstance(g.model, torch.nn.Sequential) and len(g.model) == 36
 
 
+def _seeded_like_reference(module, seed, golden):
+    """seeded_parameters_(module, seed), checked to give the drop-in exactly the reference's state_dict: the same keys
+    and shapes (what a strict load_state_dict checks) and, key by key, the same values (per-tensor sums of the
+    reference module seeded alike, stored by tests/golden/make_golden.py)."""
+    seeded_parameters_(module, seed)
+    sd = module.state_dict()
+    schema = json.loads(str(golden["sd_schema"]))
+    assert {k: list(v.shape) for k, v in sd.items()} == schema
+    np.testing.assert_allclose([sd[k].double().sum().item() for k in schema], golden["sd_sums"], rtol=1e-9, atol=1e-12)
+    return module
+
+
 def test_module_torch_composition_matches_reference_on_cpu():
-    """Feature-fallback path (CPU tensors / unsupported options) is the reference's operator sequence."""
-    from oracle import ref_import
-    if not ref_import.available():
-        pytest.skip("reference tree not present")
-    ffc = ref_import.load_reference_ffc()
+    """Feature-fallback path (CPU tensors / unsupported options) is the reference's operator sequence: the reference
+    FFC_BN_ACT's outputs on the same weights and inputs are stored in the golden."""
+    a, _ = load_golden("surface_ffcbnact_32_k3_lfu_8x8")
     kw = dict(in_channels=32, out_channels=32, kernel_size=3, ratio_gin=0.75, ratio_gout=0.75, padding=1,
               activation_layer=torch.nn.ReLU, enable_lfu=True)
-    ref = seeded_parameters_(ffc.FFC_BN_ACT(**kw).eval(), 5)
-    ours = M.FFC_BN_ACT(**kw).eval()
-    ours.load_state_dict(ref.state_dict(), strict=True)
-    xl, xg = torch.randn(1, 8, 8, 8), torch.randn(1, 24, 8, 8)
+    ours = _seeded_like_reference(M.FFC_BN_ACT(**kw).eval(), 5, a)
     with torch.no_grad():
-        a, b = ref((xl, xg)); c, d = ours((xl, xg))
-    assert torch.allclose(a, c, atol=1e-6) and torch.allclose(b, d, atol=1e-6)
+        c, d = ours((torch.from_numpy(a["x_l"]), torch.from_numpy(a["x_g"])))
+    assert torch.allclose(torch.from_numpy(a["y_l"]), c, atol=1e-6)
+    assert torch.allclose(torch.from_numpy(a["y_g"]), d, atol=1e-6)
 
 
 def test_discriminator_surface_matches_reference():
-    """FFCNLayerDiscriminator (ffc.py:370-433, training only) keeps the reference's state_dict and outputs."""
-    from oracle import ref_import
-    if not ref_import.available():
-        pytest.skip("reference tree not present")
-    ffc = ref_import.load_reference_ffc()
+    """FFCNLayerDiscriminator (ffc.py:370-433, training only) keeps the reference's state_dict and outputs (the
+    reference's output and intermediate features on the same weights and input are stored in the golden)."""
+    a, _ = load_golden("surface_discriminator_ndf16_32x32")
     kw = dict(input_nc=3, ndf=16, n_layers=3, init_conv_kwargs=dict(ratio_gin=0, ratio_gout=0.5, enable_lfu=False),
               conv_kwargs=dict(ratio_gin=0.5, ratio_gout=0.5, enable_lfu=False))
-    ref = seeded_parameters_(ffc.FFCNLayerDiscriminator(**kw).eval(), 9)
-    ours = M.FFCNLayerDiscriminator(**kw).eval()
-    ours.load_state_dict(ref.state_dict(), strict=True)
-    x = torch.randn(1, 3, 32, 32, generator=torch.Generator().manual_seed(1))
+    ours = _seeded_like_reference(M.FFCNLayerDiscriminator(**kw).eval(), 9, a)
+    fa = [torch.from_numpy(a[k]) for k in sorted(k for k in a if k.startswith("feat"))]
     with torch.no_grad():
-        a, fa = ref(x)
-        b, fb = ours(x)
-    assert torch.allclose(a, b, atol=1e-6) and len(fa) == len(fb)
+        b, fb = ours(torch.from_numpy(a["x"]))
+    assert torch.allclose(torch.from_numpy(a["y"]), b, atol=1e-6) and len(fa) == len(fb)
     assert all(torch.allclose(p, q, atol=1e-6) for p, q in zip(fa, fb))
 
 
